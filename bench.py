@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            our arm  (CUDA, through the C ABI)
   python bench.py --impl reference --gpus N ...            reference arm: the reference algorithm
                                                            restated on the box's host cores (oracle/)
+  python bench.py --steps K --warmup W --dump-outputs DIR  also writes a fixed sample of blocks of the
+                                                           last timed step's product to DIR/*.npy
 
 A "step" is one full C = A * B over the whole block matrix.  `value` is measured with the inputs
 resident in HBM; `e2e` is the same multiply through the public Dataset API with HOST buffers
@@ -334,16 +336,46 @@ def int8_peak_tops():
         return 2.0 * 1400.0, "2 x the profiling guide's sustained bf16 fallback (1.4 PFLOP/s)"
 
 
-def time_multiply(torch, stream, A, B, n, blk, steps):
+def time_multiply(torch, stream, A, B, n, blk, steps, keep_last=False):
+    """Mean ms per step over `steps` timed multiplies; with keep_last, also the product of the last step (else None)."""
     evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
-    for e0, e1 in evs:
+    last = None
+    for i, (e0, e1) in enumerate(evs):
         e0.record(stream)
         C = A.matrixMultiply(n, n, B, n, n, blk)
         e1.record(stream)
+        if keep_last and i == steps - 1:
+            last = C
         del C
     torch.cuda.synchronize()
     ms = [e0.elapsed_time(e1) for e0, e1 in evs]
-    return sum(ms) / len(ms)
+    return sum(ms) / len(ms), last
+
+
+DUMP_BUDGET_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(C, out_dir):
+    """Writes a fixed sample of the blocks of the product C, as a caller collects them, to out_dir/C_<rid>_<cid>.npy
+    (float64, numRows x numCols): the first and the last block, then blocks in an order drawn by a generator with a fixed
+    seed, as many as fit DUMP_BUDGET_BYTES in all.  The same arguments dump the same blocks.  Returns the written
+    [rid, cid] list and the bytes written."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    ids = sorted(C.block_ids())
+    order = [ids[0], ids[-1]] + [ids[k] for k in np.random.default_rng(0).permutation(len(ids))]
+    written, total = [], 0
+    for rid, cid in dict.fromkeys(order):
+        m = np.ascontiguousarray(C.get_block(rid, cid).to_numpy(), dtype=np.float64)
+        if total + m.nbytes + 128 > DUMP_BUDGET_BYTES:    # 128: the .npy header
+            if written:
+                break
+            m = np.ascontiguousarray(m[:, :max(1, (DUMP_BUDGET_BYTES - 128) // (8 * m.shape[0]))])   # one block over budget: its leading columns
+        path = os.path.join(out_dir, f"C_{rid}_{cid}.npy")
+        np.save(path, m)
+        written.append([rid, cid])
+        total += os.path.getsize(path)
+    return written, total
 
 
 def run_ours(args):
@@ -390,10 +422,15 @@ def run_ours(args):
         torch.cuda.synchronize()
         sampler.mark()
         t_wall0 = time.perf_counter()
-        ms_per_step = time_multiply(torch, stream, A, B, n, blk, args.steps)
+        ms_per_step, C_last = time_multiply(torch, stream, A, B, n, blk, args.steps, keep_last=bool(args.dump_outputs))
         t_wall = time.perf_counter() - t_wall0
         clocks = sampler.stop()
         st = s.stats()
+        dump = None
+        if args.dump_outputs:
+            blocks, nbytes = dump_outputs(C_last, args.dump_outputs)
+            dump = {"dir": args.dump_outputs, "blocks": blocks, "bytes": nbytes, "of": "C = A * B of the last timed step"}
+            del C_last
         launches_per_step = st["kernel_launches"] / args.steps
         on_tc = st["tc_gemm_launches"] > 0
 
@@ -461,7 +498,7 @@ def run_ours(args):
                     del C
                 s.sync()
                 d_steps = max(3, min(args.steps, 5))
-                d_ms = time_multiply(torch, stream, A, B, n, blk, d_steps)
+                d_ms, _ = time_multiply(torch, stream, A, B, n, blk, d_steps)
                 Cd = A.matrixMultiply(n, n, B, n, n, blk)
                 s.set_option("gemm_algo", args.algo)
                 Ct = A.matrixMultiply(n, n, B, n, n, blk)
@@ -603,6 +640,8 @@ def run_ours(args):
         "check": check,
         "dmma_fp64": dmma,
     }
+    if dump is not None:
+        line["dump_outputs"] = dump
     print(json.dumps(line), flush=True)
 
 
@@ -778,8 +817,15 @@ def main():
     ap.add_argument("--workload", default="metric", choices=("metric", "cfg5"), help="metric = BASELINE metric (dense N=16384); cfg5 = configs[4]")
     ap.add_argument("--n5", type=int, default=32768, help="matrix size of --workload cfg5")
     ap.add_argument("--pull-chunks", type=int, default=4, help="N > 1: pieces the peer pull of A is cut into")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of blocks of the last step's product C to DIR/C_<rid>_<cid>.npy "
+                         "(float64, at most 64 MB in all); single-GPU metric workload")
     ap.add_argument("--_cpu-worker", dest="cpu_worker", default=None, choices=("port", "f2j"), help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "metric" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is supported for the single-GPU metric workload of --impl ours")
     if args.cpu_worker:
         return _cpu_worker_main(args.cpu_worker, args.n, args.blk, args.steps, args.warmup, args.cpu_budget)
     if args.workload == "cfg5":
